@@ -145,6 +145,22 @@ def measured_peak_hbm():
         return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_BYTES = 60e6
+
+
+def dump_outputs(path, arrays):
+    """Writes {name: float32 array} as path/<name>.npy.  Above DUMP_BYTES in all, every array keeps the same share of its
+    rows, drawn with a fixed seed and kept in order, so that two builds given the same arguments write the same rows."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    keep = min(1.0, DUMP_BYTES / max(sum(a.nbytes for a in arrays.values()), 1))
+    rng = np.random.default_rng(0x5D12)
+    for name, a in arrays.items():
+        if keep < 1.0:
+            a = a[np.sort(rng.choice(a.shape[0], int(a.shape[0] * keep), replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def cpu_reference_run(duration_ms, nvfo=8):
     """Times the reference's own blocks on the host cores.  Returns (samples_per_s, threads, kind, what)."""
     # -march=native build first (AVX-512 where the container had it); the x86-64-v3 build if that one cannot run here
@@ -479,6 +495,13 @@ def run_b200(args):
         tma_launches = fe.stat("s1_tma_launches")
         fe.set_option("time_s1", 0)
         value = world * chunk * cps * args.steps / (ms * 1e-3) / 1e6
+        if args.dump_outputs and rank == 0:
+            # what the caller received for the last chunk of the last step (the buffers of earlier chunks have been reused):
+            # each VFO's stereo audio and the spectrum lines
+            o, keep = outs_dev[(args.steps * cps - 1) % 2]
+            got = {"vfo%d_audio" % k: keep[k][: 2 * o.vfo_count[v]].view(-1, 2).cpu().numpy() for k, v in enumerate(ids)}
+            got["fft_lines"] = keep[-1][: o.fft_lines * FFT_SIZE].view(-1, FFT_SIZE).cpu().numpy()
+            dump_outputs(args.dump_outputs, got)
 
         # ---------------- end-to-end legs (host pinned in, host pinned out) ----------------
         outs_host = [make_outputs(True), make_outputs(True)]
@@ -496,7 +519,7 @@ def run_b200(args):
                 else:
                     t.array(np.float32)[:] = dev_in[k].cpu().numpy()
             hp = [t.data_ptr() for t in host_in]
-            steps = max(8, args.steps)
+            steps = args.steps
             ecps = max(1, cps // 8)
             ems, ewall, d2h = timed_loop(hp, fmt, lib.MEM_HOST, outs_host, steps, 3, ecps)
             e2e[name] = {"value": world * chunk * ecps * steps / (ewall * 1e-3) / 1e6, "unit": "MS/s", "h2d_bytes_per_step": chunk * bps * ecps,
@@ -619,7 +642,7 @@ def run_b200(args):
     c4 = None
     if args.c4 and not args.quick:
         try:
-            c4 = c4_leg(torch, dist, sb, lib, rank, world, local, max(6, min(args.steps, 12)))
+            c4 = c4_leg(torch, dist, sb, lib, rank, world, local, args.steps)
         except Exception as ex:                      # noqa: BLE001 -- a secondary leg: never take the bench line down (all ranks fail alike)
             c4 = {"workload": C4_WORKLOAD, "value": None, "error": repr(ex)}
     c3 = None
@@ -744,7 +767,11 @@ def main():
     ap.add_argument("--c3", type=int, default=1, help="1 = also time BASELINE config 3 (256-channel polyphase filter-bank channelizer) on rank 0 and report it under 'c3'")
     ap.add_argument("--main-prio", type=int, default=-1, help="CUDA priority of the stream stage 1 runs on (0 = lowest; the library's own streams: B200_STREAM_PRIO)")
     ap.add_argument("--no-clocks", action="store_true", help="do not poll nvidia-smi during the timed region (diagnostic)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last chunk of the last step returned "
+                    "(vfo<k>_audio.npy: stereo audio of each VFO, fft_lines.npy: spectrum lines in dB; float32) to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

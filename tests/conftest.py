@@ -41,15 +41,6 @@ def oracle():
     return Oracle("restatement")
 
 
-@pytest.fixture(scope="session")
-def ref_oracle():
-    """The reference's own dsp headers over the restated leaf layer (only where it was built)."""
-    from oracle.oracle import Oracle, available
-    if not available("reference"):
-        pytest.skip("oracle/_ref/libsdrpp_ref.so not built (needs /root/reference)")
-    return Oracle("reference")
-
-
 _REPORT = {}
 
 

@@ -1,9 +1,11 @@
 """The golden cases: one function that drives an oracle implementation (reference-header build or plain-C
 restatement) over seeded inputs and returns {name: array}.  tools/make_golden.py runs it on the reference build
 and commits the result; tests/test_oracle.py runs it on the restatement and demands bit-identical arrays."""
+import hashlib
+
 import numpy as np
 
-from util import noise_iq, fm_carrier, am_carrier, ssb_tone, rds_baseband, rds_mpx_iq
+from util import noise_iq, fm_carrier, am_carrier, ssb_tone, rds_baseband, rds_mpx_iq, rds_group_bits
 
 FS = 2.4e6
 
@@ -153,3 +155,118 @@ def run_cases(R):
     g["export_i32_head"] = R.export_convert(a[:64], 2)
     g["export_u8_head"] = R.export_convert(np.clip(a[:64], -1.0, 1.0), 0)
     return g
+
+
+# ---- the block-by-block cases of test_oracle_vs_ref.py: tools/make_golden.py stores a SHA-256 of every output of the
+# reference build, the tests recompute them on the restatement.  Each function returns {name: array}.
+
+def sha256(a):
+    """bit-exact fingerprint of an array: dtype, shape and bytes"""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode())
+    h.update(a.tobytes())
+    return np.frombuffer(h.digest(), np.uint8).copy()
+
+
+def vs_ref_blocks(O, seed):
+    n = 120000
+    x = (noise_iq(n, seed, 0.3) + fm_carrier(n, FS, 300e3)).astype(np.complex64).view(np.float32)
+    mk = [
+        (lambda o: o.xlator(-300e3, FS), 12000), (lambda o: o.decim(2), 7777), (lambda o: o.decim(16), 12000),
+        (lambda o: o.decim(128), 12000), (lambda o: o.resamp(FS, 250e3), 12000), (lambda o: o.resamp(FS, 24e3), 12000),
+        (lambda o: o.resamp(48e3, 250e3), 3000), (lambda o: o.rxvfo(FS, 250e3, 150e3, 300e3), 12000),
+        (lambda o: o.rxvfo(FS, 250e3, 250e3, -123456.0), 11999), (lambda o: o.rxvfo(FS, 15e3, 10e3, 1e5), 12000),
+        (lambda o: o.dcblock_c(50.0 / FS), 12000),
+    ]
+    g = {"iq%02d" % k: f(O).process_chunks(x, ch) for k, (f, ch) in enumerate(mk)}
+    y = O.rxvfo(FS, 250e3, 150e3, 300e3).process_chunks(x, 12000)
+    g["vfo_in"] = y
+    # RDS side output of BroadcastFM (rdsOut), mono branch
+    g["wfm_rds"] = O.wfm_rds(75e3, 250e3).process_chunks(y, 1250)
+    mk2 = [
+        (lambda o: o.quad(75e3, 250e3), 1250), (lambda o: o.wfm(75e3, 250e3), 1250), (lambda o: o.wfm(75e3, 250e3, False, False), 999),
+        (lambda o: o.nfm(250e3, 12500.0, True), 1250), (lambda o: o.am(1, 10e3, 2e-4, 2e-5, 4e-4, 250e3), 1250),
+        (lambda o: o.am(0, 10e3, 2e-4, 2e-5, 4e-4, 250e3), 1250), (lambda o: o.ssb(0, 2800.0, 250e3, 2e-4, 2e-5), 1250),
+        (lambda o: o.ssb(1, 2800.0, 250e3, 2e-4, 2e-5), 1250), (lambda o: o.ssb(2, 4600.0, 250e3, 2e-4, 2e-5), 1250),
+        (lambda o: o.deemph(50e-6, 48e3), 480), (lambda o: o.resamp_stereo(250e3, 48e3), 1250),
+        (lambda o: o.wfm(75e3, 250e3, True, True), 1250), (lambda o: o.wfm(75e3, 250e3, True, False), 777),      # stereo branch: pilot PLL
+        (lambda o: o.squelch(-20.0), 1250), (lambda o: o.squelch(-60.0), 999),
+        # IF chain of the radio module (radio_module.h:90-96): noise blanker, FM IF noise reduction at its four presets
+        (lambda o: o.noise_blanker(500.0 / 24000.0, 2.0), 1250), (lambda o: o.noise_blanker(500.0 / 250e3, 1.2), 999),
+        (lambda o: o.fm_if(32), 1250), (lambda o: o.fm_if(9), 999), (lambda o: o.fm_if(15), 1250), (lambda o: o.fm_if(31), 640),
+    ]
+    for k, (f, ch) in enumerate(mk2):
+        g["vfo%02d" % k] = f(O).process_chunks(y, ch)
+    return g
+
+
+def vs_ref_design(O):
+    g = {}
+    for k, a in enumerate(((15000.0, 4000.0, 250000.0, False), (5000.0, 500.0, 15000.0, False), (3125.0, 312.5, 50000.0, True))):
+        g["lowpass%d" % k] = O.lowpass(*a)
+    g["highpass"] = O.highpass(300.0, 100.0, 48000.0)
+    g["bandpass_c"] = O.bandpass_c(18750, 19250, 3000, 250000, True).view(np.float32)
+    for r in (2, 4, 8, 16, 32, 64, 128, 256, 512, 1024, 2048, 4096, 8192):
+        plan = O.decim_plan(r)
+        g["decim_plan_%d" % r] = np.array(plan, np.int64).reshape(-1)
+        for st in range(len(plan)):
+            g["decim_taps_%d_%d" % (r, st)] = O.decim_taps(r, st)
+    for rates in ((2.4e6, 250e3), (100e6, 250e3), (1.024e9, 50e3), (8e6, 24e3), (44100.0, 48000.0)):
+        p = O.resamp_plan(*rates)
+        g["resamp_plan_%g_%g" % rates] = np.array([p[k] for k in ("mode", "predec_ratio", "interp", "decim", "ntaps", "taps_per_phase")], np.int64)
+        g["resamp_taps_%g_%g" % rates] = O.resamp_taps(*rates)
+    x = noise_iq(65536, 7, 1.0)
+    for N, nz, w in ((1024, 1024, 0), (65536, 65536, 2), (4096, 3000, 1)):
+        g["fft_%d_%d_%d" % (N, nz, w)] = O.fft_frame(N, nz, w, x[:nz])
+    line = O.fft_frame(65536, 65536, 2, x)
+    for args in ((0, 65536, 1000), (1000, 60000, 1280), (60000, 8000, 777)):
+        g["zoom_%d_%d_%d" % args] = O.zoom(args[0], args[1], args[2], line)
+    return g
+
+
+def vs_ref_formats(O):
+    """compressed sample stream (sample_stream_compressor.h / _decompressor.h) and the recorder conversions"""
+    g = {}
+    x = (noise_iq(5000, 3, 0.4) + fm_carrier(5000, FS, 300e3)).astype(np.complex64)
+    for t in (0, 1, 2):
+        g["pcm_packet%d" % t] = O.pcm_compress(x, t)
+        g["pcm_roundtrip%d" % t] = O.pcm_decompress(g["pcm_packet%d" % t]).view(np.uint32)
+    a = np.array([0.0, 0.5, -0.5, 1.0, -1.0, 2.0, -2.0, 1.5e-5, 0.25000763], np.float32)
+    for t in (0, 1, 2):
+        g["export%d" % t] = O.export_convert(a[:5] if t == 0 else a, t)
+    return g
+
+
+def vs_ref_rds_demod(O):
+    """RDSDemod: tap sets, then soft values and bits across chunk sizes and a reset"""
+    bp, bank = O.rds_demod_taps()
+    g = {"bandpass_taps": bp.view(np.float32), "interp_bank": bank}
+    x, _ = rds_baseband(3000, 11)
+    for chunk in (x.size, 839, 25, 1):
+        xs = x if chunk > 1 else x[:1500]
+        d = O.rds_demod()
+        g["soft_chunk%d" % chunk], g["hard_chunk%d" % chunk] = d.process_chunks(xs, chunk)
+        if chunk == 839:
+            d.reset()
+            g["soft_reset"], g["hard_reset"] = d.process_chunks(xs, chunk)
+    return g
+
+
+def rds_group_signal():
+    """bits of six cycles of the type-0A groups carrying PI 0xB200 / PS 'B200 DSP', and an FM carrier whose 57 kHz RDS
+    subcarrier carries them"""
+    bits = rds_group_bits(0xB200, "B200 DSP", 6)
+    x, _ = rds_mpx_iq(0, 3, bits=bits)
+    return bits, x
+
+
+def vs_ref_rds_groups(O):
+    """the RDS groups behind the rdsOut branch of BroadcastFM and RDSDemod"""
+    _, x = rds_group_signal()
+    y = O.wfm_rds(75e3, 250e3).process_chunks(x.view(np.float32), 12500)
+    soft, hard = O.rds_demod().process_chunks(y.view(np.complex64), 250)
+    return {"rds_if": y, "soft": soft, "hard": hard}
+
+
+VS_REF = {"blocks_seed1": lambda O: vs_ref_blocks(O, 1), "blocks_seed2": lambda O: vs_ref_blocks(O, 2), "design": vs_ref_design,
+          "formats": vs_ref_formats, "rds_demod": vs_ref_rds_demod, "rds_groups": vs_ref_rds_groups}

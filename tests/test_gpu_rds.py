@@ -107,12 +107,13 @@ def test_rds_demod_reads_device_memory(sb, oracle):
     assert d.process(np.empty(0, np.complex64))[0].size == 0
 
 
-@pytest.mark.xfail(strict=False, reason="added after the round's GPU minutes were spent: its first GPU run is the driver's (the same chain passes bit for bit against the oracle above)")
-def test_rds_chain_feeds_the_reference_group_decoder(sb, ref_oracle):
-    """FM carrier whose RDS subcarrier carries PI 0xB200 / PS 'B200 DSP' -> b200_wfm_rds -> b200_rds_demod -> the reference's own
-    group decoder (rds.cpp, in the reference build of the oracle): the programme identification and the name come out."""
-    from util import rds_group_bits
-    x, _ = rds_mpx_iq(0, 3, bits=rds_group_bits(0xB200, "B200 DSP", 6))
+def test_rds_chain_feeds_the_reference_group_decoder(sb):
+    """FM carrier whose RDS subcarrier carries PI 0xB200 / PS 'B200 DSP' -> b200_wfm_rds -> b200_rds_demod -> the group decoder
+    of the tests (util.rds_decode_ps, which reads from this signal what the reference's own group decoder rds.cpp read:
+    tests/test_oracle_vs_ref.py): the programme identification and the name come out."""
+    from golden_cases import rds_group_signal
+    from util import rds_decode_ps
+    _, x = rds_group_signal()
     y = sb.Block.wfm_rds(75e3, 250e3).process_chunks(x.view(np.float32), 12500).view(np.complex64)
     _, hard = sb.RdsDemod().process_chunks(y, 250)
-    assert ref_oracle.rds_group_decode(hard) == (0xB200, "B200 DSP")
+    assert rds_decode_ps(hard) == (0xB200, "B200 DSP")

@@ -3,8 +3,8 @@
 Pinning, in order of strength:
   1. golden fixtures produced by the reference's OWN dsp headers (tests/golden/reference_path.npz, made by
      tools/make_golden.py from oracle/_ref) -- the restatement must reproduce them bit for bit;
-  2. where oracle/_ref is present (the authoring container, and prebuilt on the GPU box) the restatement is compared
-     with the reference build directly on fresh random inputs (test_oracle_vs_ref.py);
+  2. SHA-256 fingerprints of the reference build's outputs, block by block on seeded random inputs
+     (tests/golden/oracle_vs_ref.npz): the restatement must match every one (test_oracle_vs_ref.py);
   3. analytic known answers (impulse -> taps, tone -> bin and level, DC gain of the decimation cascade,
      constant-frequency FM -> constant audio) and a float64 numpy FFT bound the leaf arithmetic, which is the part
      no reference artefact pins (VOLK / FFTW are external and absent: SURVEY.md section 8c).

@@ -1,87 +1,53 @@
-"""Where the reference build exists (oracle/_ref/libsdrpp_ref.so: the reference's own dsp headers over the restated
-leaf layer), the plain-C restatement must be BIT-IDENTICAL to it on fresh random inputs, block by block."""
+"""The plain-C restatement must be BIT-IDENTICAL to the reference's own dsp headers over the restated leaf layer, block by
+block.  tools/make_golden.py ran every case of golden_cases.VS_REF on the reference build and stored a SHA-256 of each output
+(dtype, shape and bytes) in tests/golden/oracle_vs_ref.npz; these tests run the same cases on the restatement."""
+import os
+
 import numpy as np
 import pytest
 
-from util import noise_iq, fm_carrier
+from golden_cases import VS_REF, rds_group_signal, sha256
+from util import rds_baseband, rds_decode_ps
 
-FS = 2.4e6
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "oracle_vs_ref.npz")
 
 
-def _same(a, b):
-    a, b = np.asarray(a), np.asarray(b)
-    return a.shape == b.shape and np.array_equal(a.view(np.uint32), b.view(np.uint32))
+@pytest.fixture(scope="module")
+def golden():
+    return np.load(GOLDEN)
+
+
+def _same_as_reference(golden, case, got):
+    want = sorted(k.split("__", 1)[1] for k in golden.files if k.startswith(case + "__") and not k.endswith(("_full", "_branch")))
+    assert sorted(got) == want
+    for name, a in got.items():
+        assert np.array_equal(sha256(a), golden[case + "__" + name]), "differs from the reference build: %s/%s" % (case, name)
 
 
 @pytest.mark.parametrize("seed", [1, 2])
-def test_blocks_bit_identical(oracle, ref_oracle, seed):
-    n = 120000
-    x = (noise_iq(n, seed, 0.3) + fm_carrier(n, FS, 300e3)).astype(np.complex64).view(np.float32)
-    R, S = ref_oracle, oracle
-    mk = [
-        (lambda o: o.xlator(-300e3, FS), 12000), (lambda o: o.decim(2), 7777), (lambda o: o.decim(16), 12000),
-        (lambda o: o.decim(128), 12000), (lambda o: o.resamp(FS, 250e3), 12000), (lambda o: o.resamp(FS, 24e3), 12000),
-        (lambda o: o.resamp(48e3, 250e3), 3000), (lambda o: o.rxvfo(FS, 250e3, 150e3, 300e3), 12000),
-        (lambda o: o.rxvfo(FS, 250e3, 250e3, -123456.0), 11999), (lambda o: o.rxvfo(FS, 15e3, 10e3, 1e5), 12000),
-        (lambda o: o.dcblock_c(50.0 / FS), 12000),
-    ]
-    for f, ch in mk:
-        assert _same(f(R).process_chunks(x, ch), f(S).process_chunks(x, ch))
-    y = R.rxvfo(FS, 250e3, 150e3, 300e3).process_chunks(x, 12000)
-    # RDS side output of BroadcastFM (rdsOut): the restatement against the reference's mono branch, and the reference's stereo
-    # branch against its mono branch (the same three blocks behind the same discriminator)
-    rds_ref = R.wfm_rds(75e3, 250e3).process_chunks(y, 1250)
-    assert abs(rds_ref.size // 2 - (y.size // 2) // 50) <= 1 and _same(rds_ref, S.wfm_rds(75e3, 250e3).process_chunks(y, 1250))
-    import ctypes as C
-    from oracle.oracle import Block
-    R.lib.orc_wfm_rds_stereo_create.restype = C.c_void_p
-    R.lib.orc_wfm_rds_stereo_create.argtypes = [C.c_double, C.c_double]
-    assert _same(Block(R.lib, R.lib.orc_wfm_rds_stereo_create(75e3, 250e3), 2, 2).process_chunks(y, 1250), rds_ref)
-    mk2 = [
-        (lambda o: o.quad(75e3, 250e3), 1250), (lambda o: o.wfm(75e3, 250e3), 1250), (lambda o: o.wfm(75e3, 250e3, False, False), 999),
-        (lambda o: o.nfm(250e3, 12500.0, True), 1250), (lambda o: o.am(1, 10e3, 2e-4, 2e-5, 4e-4, 250e3), 1250),
-        (lambda o: o.am(0, 10e3, 2e-4, 2e-5, 4e-4, 250e3), 1250), (lambda o: o.ssb(0, 2800.0, 250e3, 2e-4, 2e-5), 1250),
-        (lambda o: o.ssb(1, 2800.0, 250e3, 2e-4, 2e-5), 1250), (lambda o: o.ssb(2, 4600.0, 250e3, 2e-4, 2e-5), 1250),
-        (lambda o: o.deemph(50e-6, 48e3), 480), (lambda o: o.resamp_stereo(250e3, 48e3), 1250),
-        (lambda o: o.wfm(75e3, 250e3, True, True), 1250), (lambda o: o.wfm(75e3, 250e3, True, False), 777),      # stereo branch: pilot PLL
-        (lambda o: o.squelch(-20.0), 1250), (lambda o: o.squelch(-60.0), 999),
-        # IF chain of the radio module (radio_module.h:90-96): noise blanker, FM IF noise reduction at its four presets
-        (lambda o: o.noise_blanker(500.0 / 24000.0, 2.0), 1250), (lambda o: o.noise_blanker(500.0 / 250e3, 1.2), 999),
-        (lambda o: o.fm_if(32), 1250), (lambda o: o.fm_if(9), 999), (lambda o: o.fm_if(15), 1250), (lambda o: o.fm_if(31), 640),
-    ]
-    for f, ch in mk2:
-        assert _same(f(R).process_chunks(y, ch), f(S).process_chunks(y, ch))
+def test_blocks_bit_identical(oracle, golden, seed):
+    case = "blocks_seed%d" % seed
+    got = VS_REF[case](oracle)
+    _same_as_reference(golden, case, got)
+    # RDS side output of BroadcastFM (rdsOut): one sample per 50 of the 250 kS/s VFO; the reference's stereo branch gave the
+    # same output as its mono branch (the same three blocks behind the same discriminator)
+    assert abs(got["wfm_rds"].size // 2 - (got["vfo_in"].size // 2) // 50) <= 1
+    assert np.array_equal(golden[case + "__wfm_rds_stereo_branch"], golden[case + "__wfm_rds"])
 
 
-def test_design_and_spectrum_bit_identical(oracle, ref_oracle):
-    R, S = ref_oracle, oracle
-    for a in ((15000.0, 4000.0, 250000.0, False), (5000.0, 500.0, 15000.0, False), (3125.0, 312.5, 50000.0, True)):
-        assert _same(R.lowpass(*a), S.lowpass(*a))
-    assert _same(R.highpass(300.0, 100.0, 48000.0), S.highpass(300.0, 100.0, 48000.0))
-    assert _same(R.bandpass_c(18750, 19250, 3000, 250000, True).view(np.float32), S.bandpass_c(18750, 19250, 3000, 250000, True).view(np.float32))
-    for r in (2, 4, 8, 16, 32, 64, 128, 256, 512, 1024, 2048, 4096, 8192):
-        assert R.decim_plan(r) == S.decim_plan(r)
-        for st in range(len(R.decim_plan(r))):
-            assert _same(R.decim_taps(r, st), S.decim_taps(r, st))
-    for rates in ((2.4e6, 250e3), (100e6, 250e3), (1.024e9, 50e3), (8e6, 24e3), (44100.0, 48000.0)):
-        assert R.resamp_plan(*rates) == S.resamp_plan(*rates)
-        assert _same(R.resamp_taps(*rates), S.resamp_taps(*rates))
-    x = noise_iq(65536, 7, 1.0)
-    for N, nz, w in ((1024, 1024, 0), (65536, 65536, 2), (4096, 3000, 1)):
-        assert _same(R.fft_frame(N, nz, w, x[:nz]), S.fft_frame(N, nz, w, x[:nz]))
-    line = R.fft_frame(65536, 65536, 2, x)
-    for args in ((0, 65536, 1000), (1000, 60000, 1280), (60000, 8000, 777)):
-        assert _same(R.zoom(args[0], args[1], args[2], line), S.zoom(args[0], args[1], args[2], line))
+def test_design_and_spectrum_bit_identical(oracle, golden):
+    _same_as_reference(golden, "design", VS_REF["design"](oracle))
 
 
-def test_packet_and_export_formats_bit_identical(oracle, ref_oracle):
+def test_packet_and_export_formats_bit_identical(oracle, golden):
     """compressed sample stream (sample_stream_compressor.h / _decompressor.h) and the recorder conversions: the
     restatement against the reference's own code, plus known answers."""
-    x = (noise_iq(5000, 3, 0.4) + fm_carrier(5000, FS, 300e3)).astype(np.complex64)
+    got = VS_REF["formats"](oracle)
+    _same_as_reference(golden, "formats", got)
+    from util import noise_iq, fm_carrier
+    x = (noise_iq(5000, 3, 0.4) + fm_carrier(5000, 2.4e6, 300e3)).astype(np.complex64)
     for t in (0, 1, 2):
-        pr, ps = ref_oracle.pcm_compress(x, t), oracle.pcm_compress(x, t)
-        assert np.array_equal(pr, ps)
-        assert np.array_equal(ref_oracle.pcm_decompress(pr).view(np.uint32), oracle.pcm_decompress(ps).view(np.uint32))
+        ps = got["pcm_packet%d" % t]
         y = oracle.pcm_decompress(ps)
         # the scaler is the largest sample VALUE (not magnitude): samples inside (-max, max) come back within half a
         # step, more negative ones saturate -- the reference's behaviour, kept
@@ -93,52 +59,41 @@ def test_packet_and_export_formats_bit_identical(oracle, ref_oracle):
         assert ps.size == 8 + x.size * {0: 2, 1: 4, 2: 8}[t]
         assert int(ps[2]) + 256 * int(ps[3]) == t and int(ps[0]) == 0 and int(ps[1]) == 0
     a = np.array([0.0, 0.5, -0.5, 1.0, -1.0, 2.0, -2.0, 1.5e-5, 0.25000763], np.float32)
-    for t in (0, 1, 2):
-        assert np.array_equal(ref_oracle.export_convert(a[:5] if t == 0 else a, t), oracle.export_convert(a[:5] if t == 0 else a, t))
     assert list(oracle.export_convert(a, 1)[:7]) == [0, 16384, -16384, 32767, -32767, 32767, -32768]     # rintf: ties to even, saturation
     assert list(oracle.export_convert(a[:5], 0)) == [128, 191, 64, 255, 1]
 
 
-def test_rds_demod_bit_identical(oracle, ref_oracle):
+def test_rds_demod_bit_identical(oracle, golden):
     """RDSDemod (decoder_modules/radio/src/rds_demod.h: FastAGC, two Costas loops, band-pass, M&M clock recovery, slicer,
     differential decoder): the restatement against the reference's own class, tap sets, soft values and bits, across chunk
     sizes and a reset; the loops lock and the bits come back."""
-    from util import rds_baseband
-    bp_r, bank_r = ref_oracle.rds_demod_taps()
-    bp_s, bank_s = oracle.rds_demod_taps()
-    assert bp_r.size == 190 and _same(bp_r.view(np.float32), bp_s.view(np.float32)) and _same(bank_r, bank_s)
+    got = VS_REF["rds_demod"](oracle)
+    _same_as_reference(golden, "rds_demod", got)
     x, bits = rds_baseband(3000, 11)
+    assert got["bandpass_taps"].size == 2 * 190
     for chunk in (x.size, 839, 25, 1):
-        xs = x if chunk > 1 else x[:1500]
-        R, S = ref_oracle.rds_demod(), oracle.rds_demod()
-        sr, hr = R.process_chunks(xs, chunk)
-        ss, hs = S.process_chunks(xs, chunk)
-        assert sr.size == ss.size and abs(sr.size - xs.size * 1187.5 / 5000.0) <= 4
-        assert _same(sr, ss) and np.array_equal(hr, hs)
-        if chunk == 839:
-            R.reset(); S.reset()
-            s2, h2 = S.process_chunks(xs, chunk)
-            r2, g2 = R.process_chunks(xs, chunk)
-            assert _same(s2, r2) and np.array_equal(h2, g2)
-            # same start state after a reset, apart from the samples MM::reset leaves in its work buffer
-            assert np.array_equal(h2[8:], hs[8:])
+        n = x.size if chunk > 1 else 1500
+        assert got["soft_chunk%d" % chunk].size == got["hard_chunk%d" % chunk].size
+        assert abs(got["soft_chunk%d" % chunk].size - n * 1187.5 / 5000.0) <= 4
+    # same start state after a reset, apart from the samples MM::reset leaves in its work buffer
+    assert np.array_equal(got["hard_reset"][8:], got["hard_chunk839"][8:])
     # the decoded stream carries the transmitted bits (after the loops have settled), at some fixed delay
-    S = oracle.rds_demod()
-    _, hard = S.process_chunks(x, 1000)
+    _, hard = oracle.rds_demod().process_chunks(x, 1000)
     tail = hard[600:]
     best = max(np.mean(tail[: 2000] == bits[d: d + 2000]) for d in range(560, 640))
     assert best > 0.99, best
 
 
-def test_rds_bits_are_what_the_reference_group_decoder_reads(oracle, ref_oracle):
+def test_rds_bits_are_what_the_reference_group_decoder_reads(oracle, golden):
     """An RDS subcarrier carrying four type-0A groups (PI 0xB200, PS name 'B200 DSP', checkwords per IEC 62106) on an FM
-    carrier -> rdsOut branch -> RDSDemod (restatement, and the reference's own class) -> the reference's OWN group decoder
-    (decoder_modules/radio/src/rds.cpp, compiled from where it lies) finds the PI code and the name."""
-    from util import rds_mpx_iq, rds_group_bits
-    bits = rds_group_bits(0xB200, "B200 DSP", 6)
-    assert ref_oracle.rds_group_decode(bits) == (0xB200, "B200 DSP")               # the generator builds valid blocks
-    x, _ = rds_mpx_iq(0, 3, bits=bits)
-    for O in (oracle, ref_oracle):
-        y = O.wfm_rds(75e3, 250e3).process_chunks(x.view(np.float32), 12500).view(np.complex64)
-        _, hard = O.rds_demod().process_chunks(y, 250)
-        assert ref_oracle.rds_group_decode(hard) == (0xB200, "B200 DSP")
+    carrier -> rdsOut branch -> RDSDemod: the restatement's bits are the reference's, from which the reference's OWN group
+    decoder (decoder_modules/radio/src/rds.cpp) read the PI code and the name; the group decoder of the tests reads the same."""
+    bits, _ = rds_group_signal()
+    got = VS_REF["rds_groups"](oracle)
+    _same_as_reference(golden, "rds_groups", got)
+    assert np.array_equal(got["hard"], golden["rds_groups__hard_full"])
+    assert np.array_equal(got["soft"].view(np.uint32), golden["rds_groups__soft_full"].view(np.uint32))
+    for what, b in (("generator", bits), ("chain", got["hard"])):
+        want = (int(golden["rds_decoder__%s_pi" % what]), str(golden["rds_decoder__%s_ps" % what]))
+        assert want == (0xB200, "B200 DSP"), (what, want)
+        assert rds_decode_ps(b) == want, what

@@ -95,6 +95,34 @@ def rds_checkword(info16, offset):
     return (reg & 0x3FF) ^ offset
 
 
+RDS_OFFSET_WORDS = {0x0FC: "A", 0x198: "B", 0x168: "C", 0x350: "C'", 0x1B4: "D"}
+
+
+def rds_decode_ps(bits):
+    """Programme identification and service name from an RDS bit stream, per IEC 62106 without error correction: a group
+    counts where four consecutive 26-bit blocks carry the offset words A, B, C (or C'), D; type-0 groups give the name two
+    characters at a time.  Returns (PI or None, the 8-character name or None while a segment is missing)."""
+    b = np.asarray(bits, np.int64)
+
+    def block(p):
+        w = int("".join(map(str, b[p:p + 26])), 2)
+        info = w >> 10
+        return info, RDS_OFFSET_WORDS.get(rds_checkword(info, 0) ^ (w & 0x3FF))
+
+    pi, segs, p = None, {}, 0
+    while p + 104 <= b.size:
+        blocks = [block(p + 26 * k) for k in range(4)]
+        if [t for _, t in blocks] in (["A", "B", "C", "D"], ["A", "B", "C'", "D"]):
+            pi = blocks[0][0]
+            if blocks[1][0] >> 12 == 0:
+                segs[blocks[1][0] & 3] = blocks[3][0]
+            p += 104
+        else:
+            p += 1
+    name = "".join(chr(segs[s] >> 8) + chr(segs[s] & 0xFF) for s in range(4)) if len(segs) == 4 else None
+    return pi, name
+
+
 def rds_group_bits(pi, ps_name, repeats):
     """bit stream of `repeats` cycles of the four type-0A groups that carry the 8-character programme service name"""
     OFF = {"A": 0x0FC, "B": 0x198, "C": 0x168, "D": 0x1B4}
